@@ -281,8 +281,53 @@ def make_worker(workload, games, sims, filters, blocks, K, rank, seed, skip_stre
     return w
 
 
-def measure(args, workload, steps, warmup, world, rank, local, dist, want_e2e=True, sample_clocks=True):
-    """Device-resident timing (+ optional end-to-end timing) of one workload; returns a dict (rank 0) or None."""
+DUMP_LIMIT_BYTES = 64 << 20
+NPY_HEADER_BYTES = 128          # np.save's header for these arrays (format 1.0, padded to 64 bytes; shapes of <= 3 numbers)
+
+
+def dump_outputs(eng, out_dir, last_step, records, seed=0):
+    """Writes what a caller of the timed path (Engine.selfplay, one move of every game) holds after its last step, as
+    float64 .npy files: the step's (simulations, games finished); the games that step finished (finished_games: game
+    index, plies, value for red, flags; finished_moves: their moves as cz move codes, -1 past the last ply); and per game
+    the root position the move led to, the simulations its search ran, and the visit counts of the new root's moves.
+    Everything stays within DUMP_LIMIT_BYTES: beyond it a seeded sample of the games (indices in game_index.npy) and of the
+    finished games is written."""
+    import numpy as np
+    from cczero_b200 import records as rec
+    from cczero_b200.env import move_to_u16
+    rng = np.random.default_rng(seed)
+    stage = rec.RootStage(eng)
+    visits, moves, counts = eng.download_root_stats(stage)
+    per_game = {"root_boards": eng.download_roots(stage), "root_visits": visits, "root_moves": moves, "root_move_counts": counts,
+                "sims_run": stage.sims, "active": eng.active_flags()}
+    per_game = {k: np.asarray(v, dtype=np.float64).reshape(eng.n_games, -1) for k, v in per_game.items()}
+    plies = eng.cfg.max_plies
+    records = sorted(records, key=lambda r: r["game_index"])   # the ring's order follows the warps' finishing race
+    fin = np.array([[r["game_index"], r["n_plies"], r["value_red"], r["flags"]] for r in records], dtype=np.float64).reshape(-1, 4)
+    fin_moves = np.full((len(records), plies), -1.0)
+    for i, r in enumerate(records):
+        fin_moves[i, :len(r["moves"])] = [move_to_u16(m) for m in r["moves"]]
+    budget = DUMP_LIMIT_BYTES - (len(per_game) + 4) * NPY_HEADER_BYTES - 2 * 8
+    rec_bytes = (4 + plies) * 8
+    if len(records) * rec_bytes > budget // 2:                 # finished games get at most half of the budget
+        keep = np.sort(rng.choice(len(records), budget // 2 // rec_bytes, replace=False))
+        fin, fin_moves = fin[keep], fin_moves[keep]
+    budget -= fin.nbytes + fin_moves.nbytes
+    game_bytes = sum(v[0].nbytes for v in per_game.values()) + 8  # + its entry in game_index
+    idx = np.arange(eng.n_games)
+    if eng.n_games * game_bytes > budget:
+        idx = np.sort(rng.choice(eng.n_games, budget // game_bytes, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    out = {"last_step": np.asarray(last_step, dtype=np.float64), "finished_games": fin, "finished_moves": fin_moves,
+           "game_index": idx.astype(np.float64)}
+    out.update({k: v[idx] for k, v in per_game.items()})
+    for k, v in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+
+
+def measure(args, workload, steps, warmup, world, rank, local, dist, want_e2e=True, sample_clocks=True, dump_dir=None):
+    """Device-resident timing (+ optional end-to-end timing) of one workload; returns a dict (rank 0) or None.
+    dump_dir: where rank 0 writes the outputs of the last timed step (dump_outputs)."""
     import torch
     from cczero_b200 import records as rec
     from cczero_b200.lib import get_lib
@@ -305,10 +350,12 @@ def measure(args, workload, steps, warmup, world, rank, local, dist, want_e2e=Tr
         torch.cuda.synchronize()
 
     gather_ev = []
+    last_records = []                   # the finished-game records of the latest step (rank 0)
 
     def step_device(warm=False):
         g, s = eng.selfplay(target_games=0, max_moves=1)
         n_rec = 0
+        last_records.clear()
         if world > 1:          # the ONE collective of the path: finished-game rings -> rank 0, inside the timed region
             a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             a.record()
@@ -317,10 +364,15 @@ def measure(args, workload, steps, warmup, world, rank, local, dist, want_e2e=Tr
             gather_ev.append((a, b))
             n_rec = total
             if recs:
+                last_records.extend(rc for r, rc in recs)
                 for r, rc in recs:
                     if not (rc["flags"] & 4):
                         worker.games_stored += 1
                         worker.save_play_data(worker.games_stored, rec.record_to_play_data(rc))
+        elif g:
+            # one GPU: nothing else empties the finished-game ring, and cz_selfplay plays no move while the ring could
+            # overflow; draining it keeps every step one move of every game
+            last_records.extend(eng.drain_records())
         return s, g, n_rec
 
     for _ in range(warmup):
@@ -336,6 +388,7 @@ def measure(args, workload, steps, warmup, world, rank, local, dist, want_e2e=Tr
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     sims_total, games_done, gathered = 0, 0, 0
+    s = g = 0
     for _ in range(steps):
         s, g, nr = step_device()
         sims_total += s
@@ -346,6 +399,8 @@ def measure(args, workload, steps, warmup, world, rank, local, dist, want_e2e=Tr
     ms = e0.elapsed_time(e1)
     launches = eng.launch_count() - launches0
     st1, c1 = eng.search_stats(), eng.counters()
+    if dump_dir and rank == 0:          # after the counters: its own kernel launches are not the timed path's
+        dump_outputs(eng, dump_dir, (s, g), last_records, args.seed)
     gather_ms = sum(a.elapsed_time(b) for a, b in gather_ev)
     # ---- roofline region: the same steps with CUDA events bracketing every residual-tower launch group.  Events cannot live
     # inside the WHILE graph, so while cz_nn_profile is on the engine runs the same iteration as three sub-graphs (tree + first
@@ -451,15 +506,15 @@ def policy_bytes_per_leaf(legal):
 
 def uci_latency_block():
     """Single-game latency path (SURVEY §8f rank 4): `go depth 8` (800 simulations, search_threads 10) through the drop-in
-    `CChessPlayer(uci=True)` on the reference's trained 192x10 weights (committed fixture), wall clock around `action()`, with the
+    `CChessPlayer(uci=True)` on the reference's trained 192x10 weights (as the committed fixture rebuilds them), wall clock around `action()`, with the
     nps figure the REFERENCE's formula gives (agent/player.py:446-447).  tools/bench_uci.py is the measurement."""
     try:
         import importlib.util
         spec = importlib.util.spec_from_file_location("bench_uci", os.path.join(ROOT, "tools", "bench_uci.py"))
         mod = importlib.util.module_from_spec(spec)
         spec.loader.exec_module(mod)
-        if not os.path.exists(os.path.join(ROOT, "tests", "golden", "model_best_192x10.npz")):
-            return {"error": "tests/golden/model_best_192x10.npz missing"}
+        if not os.path.exists(os.path.join(ROOT, "tests", "golden", "model_best_192x10_compact.npz")):
+            return {"error": "tests/golden/model_best_192x10_compact.npz missing"}
         weights, src = mod.load_weights(192, 10)
         keep = os.environ.get("CZ_SEARCH_LOOP")
         try:
@@ -489,7 +544,7 @@ def run_ours(args):
     if world > 1:
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
 
-    main = measure(args, args.workload, args.steps, args.warmup, world, rank, local, dist)
+    main = measure(args, args.workload, args.steps, args.warmup, world, rank, local, dist, dump_dir=args.dump_outputs)
     secondary = {}
     if world == 1 and not args.no_secondary and args.workload == "c3":
         # BASELINE.json configs[1] and configs[4], short, each with its own roofline (driver-visible; VERDICT r1 item 4)
@@ -540,7 +595,11 @@ def main():
     ap.add_argument("--no-secondary", action="store_true", help="skip the short c2 / c5 runs (and the c1 / free-NN legs of the CPU arm)")
     ap.add_argument("--skip-stream", default="auto", choices=["auto", "fp32", "fp16"],
                     help="precision of the residual skip stream (auto = fp32 beyond 10 blocks: keeps the 1e-3 parity bound)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (float64, at most 64 MB) for comparing two builds")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference_arm(args)
     return run_ours(args)

@@ -32,6 +32,28 @@ def keras_names(filters, blocks):
     return names
 
 
+def load_compact(path):
+    """The network a compact weight file describes (written by oracle/gen_golden_weights.py): tensors stored whole
+    ("exact.<name>") are returned as they are; the large ones are regenerated from their per-output-channel mean and
+    standard deviation ("mean.", "std.", "shape.<name>") with a generator seeded by the tensor's name, and carry their
+    real first values ("head.<name>").  Names use '__' for '/'."""
+    import zlib
+    with np.load(path) as z:
+        d = {k: z[k] for k in z.files}
+    w = {}
+    for key, v in d.items():
+        kind, name = key.split(".", 1)
+        if kind == "exact":
+            w[name.replace("__", "/")] = v.astype(np.float32)
+        elif kind == "shape":
+            rng = np.random.default_rng(zlib.crc32(name.encode()))
+            a = rng.standard_normal(tuple(int(x) for x in v), dtype=np.float32) * d["std." + name] + d["mean." + name]
+            head = d["head." + name]
+            a.reshape(-1)[:head.size] = head
+            w[name.replace("__", "/")] = a.astype(np.float32)
+    return w
+
+
 def _glorot(rng, shape, fan_in, fan_out):
     lim = math.sqrt(6.0 / (fan_in + fan_out))
     return rng.uniform(-lim, lim, size=shape).astype(np.float32)

@@ -1,7 +1,8 @@
-"""Import the real reference (read-only, /root/reference) when it is present.
+"""Import the real reference: from its source tree (CZ_REFERENCE_ROOT) when that is present, else from the
+byte-compiled modules `oracle/build_ref.py` wrote into oracle/_ref (sourceless imports of the same code).
 
-Used only to validate the restatements in this directory and to generate tests/golden/.  The
-reference tree does not exist on the GPU box; callers must handle `available() == False`.
+Used only to validate the restatements in this directory and to generate tests/golden/; callers must handle
+`available() == False`.  The generators also read the reference's data files and need `source_available()`.
 Recipe from SURVEY.md Appendix B: PYTHONPATH root + the package dir itself (config.py does
 `import configs.mini`), data/log dirs redirected to a scratch directory.
 """
@@ -12,8 +13,23 @@ import tempfile
 REF_ROOT = os.environ.get("CZ_REFERENCE_ROOT", "/root/reference")
 
 
-def available():
+REF_BUILD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref")
+
+
+def source_available():
     return os.path.isdir(os.path.join(REF_ROOT, "cchess_alphazero", "environment"))
+
+
+def build_available():
+    return os.path.exists(os.path.join(REF_BUILD, "cchess_alphazero", "environment", "static_env.pyc"))
+
+
+def available():
+    return source_available() or build_available()
+
+
+def import_root():
+    return REF_ROOT if source_available() else REF_BUILD
 
 
 _done = False
@@ -24,12 +40,13 @@ def setup():
     if _done:
         return
     if not available():
-        raise RuntimeError("reference tree not present at " + REF_ROOT)
+        raise RuntimeError("reference not present: neither its source tree nor oracle/_ref")
     sys.dont_write_bytecode = True
     scratch = tempfile.mkdtemp(prefix="cz_ref_")
     os.environ.setdefault("PROJECT_DIR", scratch)
     os.environ.setdefault("DATA_DIR", os.path.join(scratch, "data"))
-    for p in (REF_ROOT, os.path.join(REF_ROOT, "cchess_alphazero")):
+    root = import_root()
+    for p in (root, os.path.join(root, "cchess_alphazero")):
         if p not in sys.path:
             sys.path.insert(0, p)
     _done = True

@@ -31,6 +31,37 @@ class FakeNetServer:
         self.stop = True
 
 
+class FairLock:
+    """A first-come-first-served lock.  The real player's sender thread sleeps while holding its queue lock and takes it
+    again right after releasing it (player.py:113-123); with the runtime's unfair locks a search thread waiting for that
+    lock can starve for as long as the host's thread wake-up latency keeps losing the race.  Served in arrival order, every
+    waiter gets the lock after at most one more sender turn; the search's results do not depend on it."""
+
+    def __init__(self):
+        self._cond = threading.Condition(threading.Lock())
+        self._next = 0
+        self._serving = 0
+
+    def acquire(self, blocking=True, timeout=-1):
+        with self._cond:
+            ticket = self._next
+            self._next += 1
+            while ticket != self._serving:
+                self._cond.wait()
+        return True
+
+    def release(self):
+        with self._cond:
+            self._serving += 1
+            self._cond.notify_all()
+
+    def __enter__(self):
+        return self.acquire()
+
+    def __exit__(self, *exc):
+        self.release()
+
+
 def make_config(sims, search_threads=1, **over):
     cfg = ref_import.config("mini")
     pc = cfg.play
@@ -49,6 +80,7 @@ def real_player_moves(states_and_opts, sims, seed, search_threads=1, use_history
     srv = FakeNetServer()
     np.random.seed(seed)
     player = pm.CChessPlayer(cfg, pipes=srv.you, enable_resign=False, use_history=use_history)
+    player.q_lock = FairLock()          # before any search runs; the sender and receiver pick it up on their next turn
     out = []
     try:
         for call in states_and_opts:

@@ -1,41 +1,63 @@
-"""Pin the oracle restatements to the REAL reference (read-only tree at /root/reference).  These tests run in the build
-container; on the GPU box the tree is absent and they skip — the committed golden vectors (tests/golden/, generated from
-the same reference by oracle/gen_golden*.py) carry the pin there."""
+"""Pin the oracle restatements to the REAL reference.  The reference's answers on the inputs below were recorded by
+oracle/gen_golden_pins.py into tests/golden/reference_pins.json.gz / .npz, so every comparison runs on any checkout.  The
+tests that execute the reference's own code around the drop-in (its model API, game loops, UCI front end and player) import
+it from its tree or from the byte-compiled modules build() leaves in oracle/_ref, and skip only where neither exists."""
+import gzip
+import json
+import os
 import random
 
 import numpy as np
 import pytest
 
+from oracle import gen_golden_pins as gen_pins
 from oracle import player as op
 from oracle import ref_import
 from oracle import senv as o
 
-pytestmark = pytest.mark.skipif(not ref_import.available(), reason="reference tree not present")
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+needs_reference = pytest.mark.skipif(not ref_import.available(), reason="runs the reference's own code: neither its tree nor "
+                                     "oracle/_ref (built by build() where the tree is present)")
 
 
-def test_env_restatement_on_random_playouts():
-    r = ref_import.senv()
-    lt = ref_import.lookup_tables()
-    assert o.ActionLabelsRed == lt.ActionLabelsRed
-    assert [o.flip_move(m) for m in o.ActionLabelsRed[:50]] == [lt.flip_move(m) for m in lt.ActionLabelsRed[:50]]
-    rng = random.Random(7)
+@pytest.fixture(scope="module")
+def pins():
+    with gzip.open(os.path.join(ROOT, "tests", "golden", "reference_pins.json.gz"), "rt") as f:
+        return json.load(f)
+
+
+@pytest.fixture(scope="module")
+def pin_arrays():
+    with np.load(os.path.join(ROOT, "tests", "golden", "reference_pins.npz")) as z:
+        return {k: z[k] for k in z.files}
+
+
+def _check_rules(row):
+    s = row["state"]
+    assert o.get_legal_moves(s) == row["legal"], s
+    assert list(o.done(s)) == row["done"] and list(o.done(s, need_check=True)) == row["done_check"], s
+    assert gen_pins.planes_digest(o.state_to_planes(s)) == row["planes"], s
+    assert o.has_attack_chessman(s) == row["attack"] and o.fliped_state(s) == row["flipped"], s
+
+
+def test_env_restatement_on_random_playouts(pins):
+    assert o.ActionLabelsRed == pins["labels"]["red"]
+    assert [o.flip_move(m) for m in o.ActionLabelsRed[:50]] == pins["labels"]["flipped_first_50"]
     n = 0
-    for g in range(25):
-        s = r.INIT_STATE
-        for ply in range(200):
-            lm = r.get_legal_moves(s)
-            assert o.get_legal_moves(s) == lm
-            assert o.done(s) == r.done(s) and o.done(s, need_check=True) == r.done(s, need_check=True)
-            assert (o.state_to_planes(s) == r.state_to_planes(s)).all()
-            assert o.has_attack_chessman(s) == r.has_attack_chessman(s) and o.fliped_state(s) == r.fliped_state(s)
-            if r.done(s)[0]:
+    for game in pins["playouts"]:
+        s = o.INIT_STATE
+        for ply, row in enumerate(game):
+            assert s == row["state"]
+            _check_rules(row)
+            if row["done"][0]:
                 break
-            m = rng.choice(lm)
+            m = row["move"]
+            assert m in row["legal"]
             if ply % 2 == 0:
-                assert o.will_check_or_catch(s, m) == r.will_check_or_catch(s, m)
-                assert o.be_catched(s, m) == r.be_catched(s, m)
-            assert o.new_step(s, m) == r.new_step(s, m)
-            s = r.step(s, m)
+                assert o.will_check_or_catch(s, m) == row["check_or_catch"]
+                assert o.be_catched(s, m) == row["catched"]
+            assert list(o.new_step(s, m)) == row["new_step"]
+            s = o.step(s, m)
             n += 1
     assert n > 500
 
@@ -50,13 +72,13 @@ def test_reference_smoke_vectors():
     assert len(o.get_legal_moves(o.INIT_STATE)) == 44
 
 
-def test_fen_helpers_match_reference():
+def test_fen_helpers_match_reference(pins):
     from cczero_b200 import env as penv
-    r = ref_import.senv()
-    s = '4s4/9/4e4/p8/2e2R2p/P5E2/8P/9/9/4S1E2'
-    for st, t in ((o.INIT_STATE, 0), (o.step(o.INIT_STATE, '0001'), 1), (s, 7), (s, 10)):
-        assert o.state_to_fen(st, t) == r.state_to_fen(st, t) == penv.state_to_fen(st, t)
-        assert o.fen_to_state(r.state_to_fen(st, t)) == r.fen_to_state(r.state_to_fen(st, t))
+    assert len(pins["fen"]) == 4
+    for row in pins["fen"]:
+        st, t = row["state"], row["turns"]
+        assert o.state_to_fen(st, t) == row["fen"] == penv.state_to_fen(st, t)
+        assert o.fen_to_state(row["fen"]) == row["state_of_fen"]
 
 
 def _oracle_root(state, sims, k, seed):
@@ -68,26 +90,26 @@ def _oracle_root(state, sims, k, seed):
     return a, pl.tree[state]
 
 
-def test_player_restatement_equals_real_player_k1():
-    from oracle.ref_player_harness import real_player_moves
-    for sims, seed in ((80, 1), (150, 2)):
-        real = real_player_moves([(o.INIT_STATE, 0, None, False)], sims, seed)[0]
-        a, node = _oracle_root(o.INIT_STATE, sims, 1, seed)
-        got = {m: (int(e.n), float(e.w), float(e.q), float(e.p)) for m, e in node.a.items()}
-        assert a == real[0] and got == real[1] and node.sum_n == real[2]
+def test_player_restatement_equals_real_player_k1(pins):
+    assert [(c["sims"], c["seed"]) for c in pins["k1_searches"]] == list(gen_pins.K1_CASES)
+    for real in pins["k1_searches"]:
+        a, node = _oracle_root(o.INIT_STATE, real["sims"], 1, real["seed"])
+        got = {m: [int(e.n), float(e.w), float(e.q), float(e.p)] for m, e in node.a.items()}
+        assert a == real["action"] and got == real["edges"] and node.sum_n == real["sum_n"]
 
 
 def test_canonical_schedule_is_statistically_the_threaded_player_k10():
     """search_threads = 10: the real player is a racy thread pool (not reproducible); the canonical schedule must be
     statistically indistinguishable from it.  Total-variation distance between root visit distributions: oracle-vs-real
-    must not exceed the real player's own run-to-run spread, and the seed-averaged distributions must agree."""
-    from oracle.ref_player_harness import real_player_moves
-    sims, k, seeds = 300, 10, range(5)
+    must not exceed the real player's own run-to-run spread, and the seed-averaged distributions must agree.  The real
+    player's distributions are the INIT_STATE row of tests/golden/mcts_k10_threaded.json.gz (oracle/gen_golden_k10.py)."""
+    with gzip.open(os.path.join(ROOT, "tests", "golden", "mcts_k10_threaded.json.gz"), "rt") as f:
+        gold = json.load(f)
+    row = next(r for r in gold["rows"] if r["state"] == o.INIT_STATE)
+    sims, k, seeds = gold["sims"], gold["search_threads"], range(5)
+    assert (sims, k) == (300, 10)
     lm = o.get_legal_moves(o.INIT_STATE)
-
-    def real(seed):
-        r = real_player_moves([(o.INIT_STATE, 0, None, False)], sims, seed, search_threads=k)[0]
-        return np.array([r[1].get(m, (0,))[0] for m in lm], float)
+    assert row["moves"] == lm
 
     def mine(seed):
         _, node = _oracle_root(o.INIT_STATE, sims, k, seed)
@@ -96,7 +118,7 @@ def test_canonical_schedule_is_statistically_the_threaded_player_k10():
     def tv(a, b):
         return 0.5 * np.abs(a / a.sum() - b / b.sum()).sum()
 
-    R, O = [real(s) for s in seeds], [mine(s) for s in seeds]
+    R, O = [np.array(row["visits"][s], float) for s in seeds], [mine(s) for s in seeds]
     assert all(x.sum() == sims - 1 for x in R + O)
     spread_real = np.mean([tv(R[i], R[j]) for i in seeds for j in seeds if i < j])
     cross = np.mean([tv(R[i], O[j]) for i in seeds for j in seeds])
@@ -104,32 +126,34 @@ def test_canonical_schedule_is_statistically_the_threaded_player_k10():
     assert tv(sum(R), sum(O)) < 0.05
 
 
-def test_game_loop_restatements_replay_live_reference_games():
+def test_game_loop_restatements_replay_live_reference_games(pins):
     """The unmodified SelfPlayWorker.start_game / EvaluateWorker.start_game (Keras/TensorFlow imports satisfied by empty
-    stand-ins, oracle/ref_worker_harness.py) against oracle/selfplay.py and oracle/arena.py, fresh seeds."""
-    import random
+    stand-ins, oracle/ref_worker_harness.py; recorded by oracle/gen_golden_pins.py) against oracle/selfplay.py and
+    oracle/arena.py, seeds of their own."""
     from oracle import arena as oarena
     from oracle import ref_worker_harness as h
     from oracle import selfplay as osp
-    play = dict(max_game_length=20, tau_decay_rate=0.98, noise_eps=0.25, enable_resign_rate=0.1, resign_threshold=-0.5, min_resign_turn=4)
+    games = pins["loop_games"]
+    assert games["play"] == gen_pins.LOOP_PLAY and games["sims"] == 16
     pc = op.PlayConfig(simulation_num_per_move=16, search_threads=1, c_puct=1.5, noise_eps=0.25, dirichlet_alpha=0.2,
                        tau_decay_rate=0.98, virtual_loss=3, resign_threshold=-0.5, min_resign_turn=4)
-    for seed in (41, 42):
-        g = h.real_selfplay_game(seed, 16, **play)
-        random.seed(seed)
-        np.random.seed(seed)
+    assert [g["seed"] for g in games["selfplay"]] == [41, 42]
+    for g in games["selfplay"]:
+        random.seed(g["seed"])
+        np.random.seed(g["seed"])
         r = osp.play_game(pc, op.fake_evaluate_states, h.ReferenceDraws(), max_game_length=20, enable_resign_rate=0.1)
         assert (r["turns"], r["value_red"], r["store"], r["final_state"]) == (g["turns"], g["value_red"], g["store"], g["final_state"])
         assert g["moves"] is None or g["moves"] == r["moves"]
-    for seed, idx in ((43, 0), (44, 1)):
-        g = h.real_arena_game(seed, idx, 16, **play)
-        random.seed(seed)
-        np.random.seed(seed)
+    assert [(g["seed"], g["idx"]) for g in games["arena"]] == [(43, 0), (44, 1)]
+    for g in games["arena"]:
+        random.seed(g["seed"])
+        np.random.seed(g["seed"])
         d = h.ReferenceDraws()
-        r = oarena.play_arena_game(pc, op.fake_evaluate_states, op.fake_evaluate_states, idx, lambda slot: d, 1, max_game_length=20)
+        r = oarena.play_arena_game(pc, op.fake_evaluate_states, op.fake_evaluate_states, g["idx"], lambda slot: d, 1, max_game_length=20)
         assert (r["turns"], r["value_red"]) == (g["turns"], g["value_red"]) and r["moves"][:len(g["moves"])] == g["moves"]
 
 
+@needs_reference
 @pytest.mark.filterwarnings("ignore::DeprecationWarning")          # api.py:68 float(array) under numpy 2
 def test_drop_in_player_searches_through_the_real_model_api(emul_lib):
     """The reference's own CChessModelAPI (agent/api.py:16-74, unmodified; a stand-in object plays the Keras model) serves
@@ -172,72 +196,67 @@ def test_drop_in_player_searches_through_the_real_model_api(emul_lib):
     player.close()
 
 
-def test_expanding_data_matches_the_real_trainer_side(emul_env):
-    """records.expanding_data vs the reference's worker/optimize.py:234-281 (unmodified; Keras imports stubbed) on one
-    golden game record, 14 and 28 planes."""
-    import gzip
-    import json
-    import os
-    from oracle import ref_worker_harness as h
-    from cczero_b200.records import expanding_data, record_to_play_data
-    h.worker_modules()
-    import cchess_alphazero.worker.optimize as ropt
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    with gzip.open(os.path.join(root, "tests", "golden", "games_k1.json.gz"), "rt") as f:
+def expanding_data_game():
+    """The first decisive self-play game of tests/golden/games_k1.json.gz, as the record record_to_play_data takes."""
+    with gzip.open(os.path.join(ROOT, "tests", "golden", "games_k1.json.gz"), "rt") as f:
         game = next(g for g in json.load(f)["games"] if g["kind"] == "selfplay" and g["result"]["moves"] and g["result"]["value_red"] != 0)
-    data = record_to_play_data({"moves": game["result"]["moves"], "value_red": game["result"]["value_red"]})
-    for use_history in (False, True):
-        rs, rp, rv = ropt.expanding_data(data, use_history)
+    return {"moves": game["result"]["moves"], "value_red": game["result"]["value_red"]}
+
+
+def test_expanding_data_matches_the_real_trainer_side(emul_env, pin_arrays):
+    """records.expanding_data vs the reference's worker/optimize.py:234-281 (unmodified; Keras imports stubbed; recorded by
+    oracle/gen_golden_pins.py) on one golden game record, 14 and 28 planes."""
+    from cczero_b200.records import expanding_data, record_to_play_data
+    data = record_to_play_data(expanding_data_game())
+    for tag, use_history in (("14", False), ("28", True)):
+        shape = tuple(pin_arrays[f"expand{tag}_states_shape"])
+        rs = np.unpackbits(pin_arrays[f"expand{tag}_states_bits"], count=int(np.prod(shape))).reshape(shape)
+        rp, rv = pin_arrays[f"expand{tag}_policy"], pin_arrays[f"expand{tag}_value"]
         s, p, v = expanding_data(data, emul_env, use_history=use_history)
         assert s.shape == rs.shape and (s == rs).all() and (p == rp).all() and (v == rv).all()
 
 
-def test_network_restatement_matches_the_shipped_keras_graph():
-    """oracle/model.py (restated from agent/model.py) vs the layer graph Keras itself wrote for the shipped networks
-    (data/model/model_best_config.json + model_best_weight.h5; model_128_l1_config.json = the 28-plane variant), executed
-    by oracle/keras_graph.py."""
-    import os
-    from cczero_b200.keras_h5 import read_keras_weights
-    from oracle import keras_graph, model as om
+def keras_graph_inputs():
+    """(192x10 weights, planes, 28-plane weights, 28-plane history planes) the Keras-graph pin runs on."""
+    from oracle import model as om
     from tests.search_checks import game_history, midgame_states
-    mdir = os.path.join(ref_import.REF_ROOT, "data", "model")
-    w = read_keras_weights(os.path.join(mdir, "model_best_weight.h5"))
+    w = om.load_compact(os.path.join(ROOT, "tests", "golden", "model_best_192x10_compact.npz"))
     states = [o.INIT_STATE] + midgame_states(11, 4, lo=2, hi=110)
     planes = np.stack([o.state_to_planes(s) for s in states])
-    gp, gv = keras_graph.run(os.path.join(mdir, "model_best_config.json"), w, planes)
-    rp, rv = om.forward(w, planes, 10)
-    assert gp.shape == (12, 2086) and np.abs(gp - rp).max() < 2e-6 and np.abs(gv[:, 0] - rv).max() < 2e-6
-    assert gp.max() > 0.2                                        # a trained, peaked policy - not a degenerate comparison
     # the 28-plane variant (Input (28,10,9), 7 blocks x 128): random weights under the names of that config
     # (that legacy file keeps the head widths of an earlier model version: 32 policy / 4 value channels)
     w28 = om.init_weights(128, 7, 256, seed=2, trained_like=True, spread=0.5, in_planes=28, policy_filters=32, value_filters=4)
     hists = [game_history(n, 30 + n) for n in (2, 5, 17, 40)]
     p28 = np.stack([o.state_history_to_planes(h[-1], h) for h in hists])
-    gp, gv = keras_graph.run(os.path.join(mdir, "model_128_l1_config.json"), w28, p28)
+    return w, planes, w28, p28
+
+
+def test_network_restatement_matches_the_shipped_keras_graph(pin_arrays):
+    """oracle/model.py (restated from agent/model.py) vs the layer graph Keras itself wrote for the shipped networks
+    (data/model/model_best_config.json with the shipped weights as tests/golden/model_best_192x10_compact.npz rebuilds
+    them; model_128_l1_config.json = the 28-plane variant), executed by oracle/keras_graph.py and recorded by
+    oracle/gen_golden_pins.py."""
+    from oracle import model as om
+    w, planes, w28, p28 = keras_graph_inputs()
+    gp, gv = pin_arrays["graph_policy"], pin_arrays["graph_value"]
+    rp, rv = om.forward(w, planes, 10)
+    assert gp.shape == (12, 2086) and np.abs(gp - rp).max() < 2e-6 and np.abs(gv[:, 0] - rv).max() < 2e-6
+    assert gp.max() > 50 / 2086                                  # a peaked policy - not a degenerate comparison
+    gp, gv = pin_arrays["graph28_policy"], pin_arrays["graph28_value"]
     rp, rv = om.forward(w28, p28, 7)
-    assert np.abs(gp - rp).max() < 2e-6 and np.abs(gv[:, 0] - rv).max() < 2e-6
+    assert gp.shape == (4, 2086) and np.abs(gp - rp).max() < 2e-6 and np.abs(gv[:, 0] - rv).max() < 2e-6
 
 
-def test_evaluator_tally_matches_the_real_worker():
-    """EvaluateWorker.start's win / draw / fail bookkeeping and score (evaluator.py:93-145, unmodified) over canned game
-    results vs cczero_b200.evaluator.tally_games."""
-    from oracle import ref_worker_harness as h
+def test_evaluator_tally_matches_the_real_worker(pins):
+    """EvaluateWorker.start's win / draw / fail bookkeeping and score (evaluator.py:93-145, unmodified; recorded by
+    oracle/gen_golden_pins.py) over canned game results vs cczero_b200.evaluator.tally_games."""
     from cczero_b200.evaluator import tally_games
-    _, ev = h.worker_modules()
-    cfg = ref_import.config("mini")
-    results = [1, -1, 0, 1, 1, -1, 0, 0, -1, 1, 1, -1]
-    cfg.eval.game_num = len(results)
-    w = ev.EvaluateWorker(cfg, pid=0)
-    w.start_game = lambda idx: (results[idx], 40)
-    sleep = ev.sleep
-    ev.sleep = lambda s: None
-    try:
-        want = w.start()
-    finally:
-        ev.sleep = sleep
-    assert tuple(want) == tuple(tally_games(list(enumerate(results))))
+    results = pins["evaluator"]["results"]
+    assert results == gen_pins.TALLY_RESULTS
+    assert list(tally_games(list(enumerate(results)))) == pins["evaluator"]["tally"]
 
 
+@needs_reference
 def test_reference_game_loops_drive_the_drop_in_player(emul_lib):
     """INTEGRATION.md §3, literally: the name `CChessPlayer` inside the reference's worker modules is rebound to
     cczero_b200.player.CChessPlayer and the UNMODIFIED SelfPlayWorker.start_game / EvaluateWorker.start_game play whole
@@ -269,6 +288,7 @@ def test_reference_game_loops_drive_the_drop_in_player(emul_lib):
     assert done >= 8
 
 
+@needs_reference
 def test_reference_uci_front_end_drives_the_drop_in_player(emul_lib):
     """The REAL uci.UCI class with `CChessPlayer` rebound to the drop-in: the golden session (recorded with the real
     player) must come out line for line."""
@@ -329,6 +349,7 @@ def test_reference_uci_front_end_drives_the_drop_in_player(emul_lib):
             s.close()
 
 
+@needs_reference
 def test_reference_player_runs_on_the_drop_in_rules_engine(emul_env):
     """The other import swap of INTEGRATION.md §3: `senv` inside the reference's agent/player.py rebound to
     cczero_b200.env.StaticEnv - the REAL player must search exactly as it does on its own static_env."""
@@ -350,17 +371,16 @@ def test_reference_player_runs_on_the_drop_in_rules_engine(emul_env):
         pm.senv = own
 
 
-def test_env_restatement_on_arbitrary_boards():
+def test_env_restatement_on_arbitrary_boards(pins):
     """Unreachable positions (random pieces on random squares, piece counts no game can have): oracle == real static_env."""
     from tests.env_checks import EXTREME_STATES, random_boards
-    r = ref_import.senv()
-    for s in random_boards(600, 5) + [x for x in EXTREME_STATES if 's' in x and 'S' in x]:
-        lm = r.get_legal_moves(s)
-        assert o.get_legal_moves(s) == lm, s
-        assert o.done(s) == r.done(s) and o.done(s, need_check=True) == r.done(s, need_check=True), s
-        assert (o.state_to_planes(s) == r.state_to_planes(s)).all() and o.has_attack_chessman(s) == r.has_attack_chessman(s)
-        if lm and not r.done(s)[0]:
-            m = lm[len(s) % len(lm)]
-            assert o.new_step(s, m) == r.new_step(s, m), (s, m)
-            assert o.will_check_or_catch(s, m) == r.will_check_or_catch(s, m), (s, m)
-            assert o.be_catched(s, m) == r.be_catched(s, m), (s, m)
+    states = random_boards(600, 5) + [x for x in EXTREME_STATES if 's' in x and 'S' in x]
+    assert [row["state"] for row in pins["arbitrary_boards"]] == states
+    for row in pins["arbitrary_boards"]:
+        s = row["state"]
+        _check_rules(row)
+        if "move" in row:
+            m = row["move"]
+            assert list(o.new_step(s, m)) == row["new_step"], (s, m)
+            assert o.will_check_or_catch(s, m) == row["check_or_catch"], (s, m)
+            assert o.be_catched(s, m) == row["catched"], (s, m)

@@ -5,7 +5,8 @@ search, simulations/s and the `nps` figure computed with the REFERENCE'S formula
 slice of the search; =graph: three sub-graphs per iteration and a polled flag) and the round-1 host-driven loop (=host).
 
     python tools/bench_uci.py [filters blocks] [depth] [search_threads]
-Weights: the reference's trained 192x10 network (tests/golden/model_best_192x10.npz) by default."""
+Weights: the reference's trained 192x10 network as tests/golden/model_best_192x10_compact.npz rebuilds it (real batch-norm
+statistics and biases, kernels of the real per-channel scale) by default."""
 import io
 import json
 import os
@@ -48,11 +49,11 @@ def run(loop, filters, blocks, depth, k, weights):
 
 
 def load_weights(filters, blocks):
-    npz = os.path.join(ROOT, "tests", "golden", "model_best_192x10.npz")
-    if (filters, blocks) == (192, 10) and os.path.exists(npz):
-        with np.load(npz) as z:
-            return {key.replace("__", "/"): torch.as_tensor(z[key]) for key in z.files}, "reference's trained 192x10 weights"
     from oracle import model as om
+    npz = os.path.join(ROOT, "tests", "golden", "model_best_192x10_compact.npz")
+    if (filters, blocks) == (192, 10) and os.path.exists(npz):
+        return ({key: torch.as_tensor(v) for key, v in om.load_compact(npz).items()},
+                "reference's trained 192x10 weights, rebuilt from tests/golden/model_best_192x10_compact.npz")
     return {key: torch.as_tensor(v) for key, v in om.init_weights(filters, blocks, 256, seed=0).items()}, "random-init weights"
 
 
